@@ -2,6 +2,7 @@
 """bench.py -- denoise-steps/sec of the PixArt-Sigma-XL/2 denoiser hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c4|c5|vae|t5] [--impl ours|reference] [--no-extras]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -30,6 +31,13 @@ CPU sample of the reference's own path (diffusers is absent: the oracle decoder;
 leaves the `fp32_attention` flag of the reference's 1024px config off (it selects the hi + lo P form of the attention forward).
 
 One JSON line is printed by rank 0.
+
+`--dump-outputs DIR` writes, after the timed steps, what the timed path handed its caller in its LAST timed step as
+`DIR/<name>.npy` (float32, rank 0): `eps` (the forward's noise prediction; `c4_eps` for the extra c4 line), `loss` and `grads`
+(the training step's mean loss and the gradients of all parameters in `named_parameters` order, flattened; `train_` prefix for
+the extra line), `stack_out` (vae) and `last_hidden_state` (t5).  An array of more than DUMP_MAX_ELEMS elements is replaced by
+the same seeded sample of its flattened elements in every run.  Weights and inputs come from fixed seeds, so two builds run
+with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -40,6 +48,7 @@ import sys
 import tempfile
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -72,6 +81,25 @@ def flops_per_forward(n_tok: int, batch: int, kv_compress: bool):
         tot_attn += 4 * n_tok * nk * C + 4 * n_tok * L * C
     emb = 2 * L * 4096 * C + 2 * L * C * C + 2 * n_tok * 16 * C + 2 * n_tok * C * 32 + (2 * 256 * C + 14 * C * C)
     return batch * (tot_gemm + tot_attn + emb), batch * (tot_gemm + 2 * L * 4096 * C + 2 * L * C * C), batch * tot_attn
+
+
+DUMP_SEED, DUMP_MAX_ELEMS, DUMP_MAX_BYTES = 0, 1 << 23, 64 << 20
+
+
+def dump_array(t: torch.Tensor) -> np.ndarray:
+    """`t` as float32 on the host; above DUMP_MAX_ELEMS elements, the DUMP_SEED-seeded sample of its flattened elements."""
+    t = t.detach()
+    if t.numel() > DUMP_MAX_ELEMS:
+        idx = torch.randint(0, t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(DUMP_SEED))
+        t = t.reshape(-1)[idx.to(t.device)]
+    return t.float().cpu().numpy()
+
+
+def write_outputs(out_dir: str, outputs: dict) -> None:
+    assert outputs and sum(a.nbytes for a in outputs.values()) <= DUMP_MAX_BYTES, {k: a.nbytes for k, a in outputs.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -127,9 +155,10 @@ class ClockSampler:
 
 # --------------------------------------------------------------------------------------------- distributed context
 class Ctx:
-    def __init__(self, gpus: int):
+    def __init__(self, gpus: int, dump: bool = False):
         import torch.distributed as dist
         self.dist = dist
+        self.last_output, self.outputs = None, {}
         self.rank, self.world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
         self.local = int(os.environ.get("LOCAL_RANK", "0"))
         if self.world == 1 and gpus > 1:
@@ -138,6 +167,12 @@ class Ctx:
         self.dev = torch.device("cuda", self.local)
         if self.world > 1:
             dist.init_process_group("nccl", device_id=self.dev)
+        self.dumping = dump and self.rank == 0
+
+    def keep(self, name: str, t: torch.Tensor) -> None:
+        """Record `t` for --dump-outputs (rank 0 only)."""
+        if self.dumping:
+            self.outputs[name] = dump_array(t)
 
     def barrier(self):
         if self.world > 1:
@@ -145,14 +180,16 @@ class Ctx:
         torch.cuda.synchronize()
 
     def timed(self, fn, steps: int) -> float:
-        """EXACTLY `steps` calls between two CUDA events, barrier + synchronize on both sides, max over ranks (ms)."""
+        """EXACTLY `steps` calls between two CUDA events, barrier + synchronize on both sides, max over ranks (ms).
+        What the last call returned is left in `last_output`."""
         self.barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(steps):
-            fn(i)
+            out = fn(i)
         e1.record()
         self.barrier()
+        self.last_output = out
         ms = e0.elapsed_time(e1)
         if self.world > 1:
             tt = torch.tensor([ms], device=self.dev)
@@ -451,6 +488,7 @@ def measure_inference(args, ctx: Ctx, wl_name: str, headline: bool):
         ms = ctx.timed(step_resident, args.steps)                                   # <- `value`: nothing else in here
         if os.environ.get("PXA_PROFILER_RANGE") == "1":
             torch.cuda.profiler.stop()
+        ctx.keep("eps" if headline else f"{wl_name}_eps", ctx.last_output)
         ms_e2e = ctx.timed(step_e2e, args.steps)
         clocks = sampler.stop() if sampler else None
         # ---- separate pass: per-kernel CUDA events for the roofline (2 steps; not part of value / e2e)
@@ -616,6 +654,10 @@ def measure_train(args, ctx: Ctx, mode: str, checkpoint: bool, cpu_baseline: boo
     t_host = time.perf_counter()
     ms = ctx.timed(step_resident, args.steps)
     host_total_ms = (time.perf_counter() - t_host) * 1000.0
+    prefix = "" if args.workload == "c5" else "train_"
+    ctx.keep(prefix + "loss", ctx.last_output)
+    if ctx.dumping:
+        ctx.keep(prefix + "grads", torch.cat([p.grad.reshape(-1) for p in model.parameters() if p.grad is not None]))
     ms_e2e = ctx.timed(step_e2e, args.steps)
     clocks = sampler.stop() if sampler else None
     # exposed part of the gradient all-reduce: the same step with the collective switched off (world > 1 only)
@@ -732,6 +774,7 @@ def measure_vae(args, ctx: Ctx):
     n0 = lib.launch_count()
     ms = ctx.timed(step, args.steps)
     launches = lib.launch_count() - n0
+    ctx.keep("stack_out", ctx.last_output)
     clocks = sampler.stop() if sampler else None
     # e2e: the call scripts/inference.py:136 makes -- `vae.decode(latent / scaling_factor).sample` of the whole autoencoder (conv_in,
     # mid block incl. its 16384-token attention, the stack above, conv_norm_out, conv_out) with the latent copied from pinned host
@@ -841,6 +884,7 @@ def measure_t5(args, ctx: Ctx):
     n0 = lib.launch_count()
     ms = ctx.timed(step, args.steps)
     launches = lib.launch_count() - n0
+    ctx.keep("last_hidden_state", ctx.last_output)
     clocks = sampler.stop() if sampler else None
     ms_e2e = ctx.timed(step_e2e, args.steps)
     timer = KernelTimer(lib, [("gemm", "gemm"), ("rms", "rmsnorm"), ("attn", "t5_attn")])
@@ -922,8 +966,14 @@ def main():
     ap.add_argument("--no-cuda-graph", dest="cuda_graph", action="store_false",
                     help="issue the forward eagerly (default: `value` and `e2e` replay it as ONE CUDA graph through the "
                          "public pixart_sigma_b200.graph.GraphedForward: ~310 launches and their host work per step disappear)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy (float32)")
     ap.set_defaults(cuda_graph=True)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path: use it with --impl ours")
     # The contract is ONE JSON line on stdout.  Libraries write banners there too (NCCL prints its version line at the
     # first communicator init), so fd 1 is pointed at stderr for the whole run and the JSON line goes to the saved fd.
     global _JSON_FD
@@ -937,7 +987,7 @@ def main():
         run_reference_arm(args, WORKLOADS[args.workload])
         return
     from pixart_sigma_b200 import lib
-    ctx = Ctx(args.gpus)
+    ctx = Ctx(args.gpus, dump=bool(args.dump_outputs))
     lib.load()
     train_mode = "graph" if args.train_mode == "auto" else args.train_mode
     if args.workload == "vae":
@@ -959,6 +1009,8 @@ def main():
                         "steps", "warmup")
                 line["train"] = {k: tr[k] for k in keep if k in tr}
                 line["c4"] = {k: c4[k] for k in keep if k in c4}
+    if ctx.dumping:
+        write_outputs(args.dump_outputs, ctx.outputs)
     if ctx.rank == 0:
         _emit(line)
     ctx.close()

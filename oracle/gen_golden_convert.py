@@ -1,7 +1,8 @@
 """TEST INFRASTRUCTURE ONLY -- run the key-mapping body of the UNMODIFIED reference converter
-(`/root/reference/tools/convert_pixart_to_diffusers.py:27-154`, exec'd on a synthetic small-width state dict with the
-reference key layout) and store what it produced: tests/golden/diffusers_mapping.pt = {diffusers key: (reference-side
-provenance checksum, shape)} for the plain, micro-condition and qk-norm variants.  Run in the build container only."""
+(`tools/convert_pixart_to_diffusers.py:27-154` of the reference checkout that oracle/refshim.py finds, exec'd on a synthetic
+small-width state dict with the reference key layout) and store what it produced: tests/golden/diffusers_mapping.pt =
+{diffusers key: (shape, sum, sum of magnitudes)} plus a position-weighted sum per key (`weighted_sum`, which a reordering inside
+a tensor changes) for the plain, micro-condition and qk-norm variants.  Needs the reference checkout."""
 import os
 import sys
 import textwrap
@@ -12,8 +13,15 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from oracle import pixart_oracle as po  # noqa: E402
+from oracle.refshim import REFERENCE_ROOT  # noqa: E402
 
-REF = "/root/reference/tools/convert_pixart_to_diffusers.py"
+REF = os.path.join(REFERENCE_ROOT, "tools", "convert_pixart_to_diffusers.py")
+
+
+def weighted_sum(v: torch.Tensor) -> float:
+    """sum_i cos(i) * v.flatten()[i] in float64: unlike the plain sums it changes when elements swap places."""
+    flat = v.detach().double().flatten()
+    return float((flat * torch.arange(flat.numel(), dtype=torch.float64).cos()).sum())
 
 
 def small_state_dict(micro: bool, qk: bool):
@@ -37,7 +45,8 @@ def main():
         sd = small_state_dict(micro, qk)
         conv, left = reference_mapping(sd, micro, qk)
         fix[name] = {"micro": micro, "qk": qk, "left_over": sorted(left),
-                     "entries": {k: (tuple(v.shape), float(v.double().sum()), float(v.double().abs().sum())) for k, v in conv.items()}}
+                     "entries": {k: (tuple(v.shape), float(v.double().sum()), float(v.double().abs().sum())) for k, v in conv.items()},
+                     "weighted_sum": {k: weighted_sum(v) for k, v in conv.items()}}
         print(name, len(conv), "converted keys,", len(left), "left over:", sorted(left))
     torch.save(fix, os.path.join(ROOT, "tests", "golden", "diffusers_mapping.pt"))
 

@@ -12,9 +12,9 @@ that restate the *published* behaviour of the few symbols the hot path touches:
   mmcv.Registry / mmcv.runner.get_dist_info / mmcv.utils.logging.logger_initialized
       (call sites: diffusion/model/builder.py:1,5,11; diffusion/utils/logger.py:6; dist_utils.py:10,13)
 
-Nothing here is imported by the product package `pixart_sigma_b200`; it is used by
-`oracle/gen_golden.py` (fixture generation, this container only) and by `-m "not gpu"` tests that
-validate `oracle/pixart_oracle.py` against the real reference when `/root/reference` exists.
+Nothing here is imported by the product package `pixart_sigma_b200`; it is used by the
+`oracle/gen_golden*.py` fixture generators, which need a reference checkout, and the registry stand-in
+by `tests/test_host_cpu.py`, which needs none.
 """
 import os
 import sys

@@ -1,7 +1,11 @@
 """CPU tests (-m "not gpu"): host-side mirror of the reference interface, C-ABI library surface, build recipe."""
 import ctypes
+import inspect
+import json
 import os
 import re
+import sys
+import types
 
 import pytest
 import torch
@@ -11,6 +15,13 @@ from oracle import refshim
 from pixart_sigma_b200 import MODELS, PixArtMS, PixArtMS_XL_2, PixArtMSBlock, build_model, lib
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+
+@pytest.fixture(scope="module")
+def reference_surface(golden_dir):
+    """What the unmodified reference exposes (tests/golden/reference_surface.json, written by oracle/gen_golden_surface.py)."""
+    with open(os.path.join(golden_dir, "reference_surface.json")) as f:
+        return json.load(f)
 
 
 def _tiny(**kw):
@@ -38,19 +49,14 @@ def test_state_dict_layout_optional_modules(kw, cfg):
     assert got == po.state_dict_shapes(po.OracleConfig(depth=2, **cfg))
 
 
-@pytest.mark.skipif(not refshim.reference_available(), reason="/root/reference not present")
-def test_state_dict_keys_equal_live_reference():
-    from oracle.gen_golden import build_reference
-    refshim.install_reference_shims()
-    cfg = po.OracleConfig(depth=1, kv_sampling="conv", kv_scale_factor=2, kv_compress_layer=[0])
-    ref = build_reference(cfg, po.synthetic_state_dict(cfg))
+def test_state_dict_keys_equal_live_reference(reference_surface):
+    ref = {k: tuple(v) for k, v in reference_surface["pixartms_d1_kvconv_state_dict"].items()}
     ours = PixArtMS(depth=1, input_size=32, model_max_length=300,
                     kv_compress_config=dict(sampling="conv", scale_factor=2, kv_compress_layer=[0]))
-    rs, os_ = ref.state_dict(), ours.state_dict()
-    assert set(rs) == set(os_)
-    assert all(rs[k].shape == os_[k].shape for k in rs)
+    os_ = {k: tuple(v.shape) for k, v in ours.state_dict().items()}
+    assert os_ == ref
     # a reference checkpoint loads with the same strict=False call the reference scripts use
-    sd = {k: v for k, v in rs.items() if k != "pos_embed"}            # scripts/inference.py:181-184
+    sd = {k: torch.randn(v) for k, v in ref.items() if k != "pos_embed"}            # scripts/inference.py:181-184
     missing, unexpected = ours.load_state_dict(sd, strict=False)
     assert missing == ["pos_embed"] and not unexpected
 
@@ -138,20 +144,32 @@ def test_product_never_imports_the_oracle():
             assert "oracle" not in open(os.path.join(pkg, fn)).read().replace("the oracle", ""), fn
 
 
-@pytest.mark.skipif(not refshim.reference_available(), reason="/root/reference not present")
-def test_install_into_reference_repoints_registry_and_nets():
+def test_install_into_reference_repoints_registry_and_nets(reference_surface, monkeypatch):
     """INTEGRATION.md level A: after install_into_reference() the reference's own builder / module names construct
-    the B200 model, so scripts/inference.py and train_scripts/train.py pick it up unchanged."""
-    refshim.install_reference_shims()
+    the B200 model, so scripts/inference.py and train_scripts/train.py pick it up unchanged.  The reference package is
+    stood in for by modules holding the names it registers and exports (tests/golden/reference_surface.json); its
+    `build_model` resolves a model name through `MODELS.build` of the mmcv registry (diffusion/model/builder.py:8-11)."""
     import pixart_sigma_b200
+    placeholder = object()
+    registry = refshim._Registry("models")
+    for name in reference_surface["registry"]:
+        registry.register_module(name=name, module=placeholder)
+    pkg, model_pkg = types.ModuleType("diffusion"), types.ModuleType("diffusion.model")
+    nets, builder = types.ModuleType("diffusion.model.nets"), types.ModuleType("diffusion.model.builder")
+    for name in reference_surface["nets"]:
+        setattr(nets, name, placeholder)
+    builder.MODELS = registry
+    pkg.model, model_pkg.nets, model_pkg.builder = model_pkg, nets, builder
+    for mod in (pkg, model_pkg, nets, builder):
+        monkeypatch.setitem(sys.modules, mod.__name__, mod)
     assert pixart_sigma_b200.install_into_reference()
-    import diffusion.model.nets as nets
-    from diffusion.model.builder import build_model as ref_build_model
-    assert nets.PixArtMS is PixArtMS and nets.PixArtMSBlock is PixArtMSBlock
-    m = ref_build_model("PixArtMS", False, False, depth=1, input_size=32, model_max_length=300)
+    assert all(getattr(nets, n) is getattr(pixart_sigma_b200, n) for n in reference_surface["nets"])
+    assert all(registry.get(n) is getattr(pixart_sigma_b200, n) for n in reference_surface["registry"])
+    m = registry.build(dict(type="PixArtMS"), default_args=dict(depth=1, input_size=32, model_max_length=300))
     assert type(m) is PixArtMS
     # the reference sampler wrapper accepts the model's bound method (diffusion/dpm_solver.py:6-36)
     from diffusion import DPMS
+    assert list(inspect.signature(DPMS).parameters) == reference_surface["dpms_params"]
     cond = torch.zeros(1, 1, 300, 4096)
     solver = DPMS(m.forward_with_dpmsolver, condition=cond, uncondition=cond, cfg_scale=4.5,
                   model_kwargs=dict(data_info=None, mask=None))
@@ -182,27 +200,22 @@ def test_hi_lo_split_of_p_carries_sixteen_mantissa_bits():
     assert 2.0 ** -9 < err1 <= 2.0 ** -8 and err2 <= 2.0 ** -17
 
 
-@pytest.mark.skipif(not refshim.reference_available(), reason="/root/reference not present")
-def test_single_scale_pixart_surface_equals_live_reference():
+def test_single_scale_pixart_surface_equals_live_reference(reference_surface):
     """nets/PixArt.py: `PixArt` / `PixArt_XL_2` / `PixArtBlock` (the 256px Sigma config builds `PixArt_XL_2`,
     configs/pixart_sigma_config/PixArt_sigma_xl2_img256_internal.py:12): same state-dict keys and shapes as the unmodified reference
-    class, registry names, the single-scale forward signatures."""
-    import inspect
+    class, registry names, the single-scale forward signatures (tests/golden/reference_surface.json)."""
     from pixart_sigma_b200 import PixArt, PixArt_XL_2, PixArtBlock
-    refshim.install_reference_shims()
-    from diffusion.model.nets.PixArt import PixArt as RefPixArt
     kv = dict(sampling="conv", scale_factor=2, kv_compress_layer=[1])
-    ref = RefPixArt(input_size=16, depth=2, model_max_length=300, qk_norm=True, kv_compress_config=kv)
     ours = PixArt(input_size=16, depth=2, model_max_length=300, qk_norm=True, kv_compress_config=kv)
-    rs, os_ = ref.state_dict(), ours.state_dict()
-    assert set(rs) == set(os_) and all(rs[k].shape == os_[k].shape for k in rs)
-    missing, unexpected = ours.load_state_dict(rs, strict=True), None
-    assert set(MODELS.module_dict) >= {"PixArt", "PixArt_XL_2"}
+    ref = {k: tuple(v) for k, v in reference_surface["pixart_single_scale_state_dict"].items()}
+    assert {k: tuple(v.shape) for k, v in ours.state_dict().items()} == ref
+    ours.load_state_dict({k: torch.randn(v) for k, v in ref.items()}, strict=True)
+    assert set(MODELS.module_dict) >= set(reference_surface["registry"])
     assert isinstance(build_model("PixArt", depth=1, input_size=8), PixArt) and callable(PixArt_XL_2)
     assert all(type(b) is PixArtBlock for b in ours.blocks) and not ours.micro_conditioning and ours.out_channels == 8
     for name in ("forward", "forward_with_dpmsolver", "forward_with_cfg"):
         ours_p = list(inspect.signature(getattr(PixArt, name)).parameters)
-        ref_p = list(inspect.signature(getattr(RefPixArt, name)).parameters)
+        ref_p = reference_surface["pixart_signatures"][name]
         assert ours_p == ref_p, (name, ours_p, ref_p)
     assert list(inspect.signature(PixArtBlock.forward).parameters)[:5] == ["self", "x", "y", "t", "mask"]
     with pytest.raises(ValueError, match="single-scale"):

@@ -1,6 +1,5 @@
 """CPU tests (-m "not gpu"): the oracle restatement against the committed golden fixtures that
-oracle/gen_golden.py produced from the UNMODIFIED reference, and -- when /root/reference is present --
-against the reference itself, live."""
+oracle/gen_golden.py and oracle/gen_golden_surface.py produced from the UNMODIFIED reference."""
 import glob
 import os
 
@@ -9,7 +8,7 @@ import pytest
 import torch
 
 from oracle import pixart_oracle as po
-from oracle import refshim
+from oracle.gen_golden_surface import ragged_inputs
 
 TOL = 2e-5  # fp32 vs fp32, different op order only
 
@@ -85,27 +84,16 @@ def test_state_dict_layout_matches_survey_counts():
     assert len(po.state_dict_shapes(kv)) == 492
 
 
-@pytest.mark.skipif(not refshim.reference_available(), reason="/root/reference not present (GPU box)")
-def test_oracle_matches_live_reference_ragged_mask():
-    """Live check against the unmodified reference with a NON-prefix 0/1 mask (masked_select semantics)."""
-    from oracle.gen_golden import build_reference
-    refshim.install_reference_shims()
-    cfg = po.OracleConfig(depth=1, input_size=32, pe_interpolation=0.5)
-    sd = po.synthetic_state_dict(cfg, seed=3)
-    x, t, y, _ = po.synthetic_inputs(cfg, 2, (16, 24), seed=3, timesteps=[749.25, 3.0])
-    mask = (torch.rand(2, 300, generator=torch.Generator().manual_seed(5)) > 0.5).long()
-    ref = build_reference(cfg, sd)
-    with torch.no_grad():
-        want = ref(x, t, y, mask=mask, data_info=None)
+def test_oracle_matches_live_reference_ragged_mask(golden_dir):
+    """Against the unmodified reference with a NON-prefix 0/1 mask (masked_select semantics); its outputs are stored in
+    tests/golden/ragged_mask_d1.pt (oracle/gen_golden_surface.py)."""
+    fix = torch.load(os.path.join(golden_dir, "ragged_mask_d1.pt"))
+    cfg, sd, x, t, y, mask = ragged_inputs()
     got = po.forward(sd, cfg, x, t, y, mask=mask)
-    assert po.rel_err(got, want) < TOL
+    assert po.rel_err(got, fix["out"]) < TOL
     # batch-broadcast 2-D mask (CFG: n masks for 2n samples, PixArtMS.py:197-198) ...
-    with torch.no_grad():
-        want2 = ref(x, t, y, mask=mask[:1], data_info=None)
     got2 = po.forward(sd, cfg, x, t, y, mask=mask[:1])
-    assert po.rel_err(got2, want2) < TOL
+    assert po.rel_err(got2, fix["out_mask_broadcast"]) < TOL
     # ... and the trainer's (B,1,1,L) layout (train.py:158-168; squeezed at PixArtMS.py:199)
-    with torch.no_grad():
-        want3 = ref(x, t, y, mask=mask.reshape(2, 1, 1, 300), data_info=None)
     got3 = po.forward(sd, cfg, x, t, y, mask=mask.reshape(2, 1, 1, 300))
-    assert po.rel_err(got3, want3) < TOL
+    assert po.rel_err(got3, fix["out_mask_b11l"]) < TOL
