@@ -342,6 +342,43 @@ typedef struct PxaDpmStepArgs {
 } PxaDpmStepArgs;
 int pxa_dpm_solver_pp_step(const PxaDpmStepArgs* args, void* stream);
 
+/* ------------------------------------------------------------------------------------ SA-Solver sampler step
+ * One fused elementwise pass per denoiser evaluation i of the SA-Solver "few steps" loop (predictor order 2, corrector
+ * order 2, PEC) the reference runs in PyTorch (diffusion/model/sa_solver.py: CFG combine :310-318, data prediction
+ * :377-386, predictor :644-698, corrector :700-753, loop :755-909; wrapper diffusion/sa_sampler.py:75-92):
+ *     eps   = eps_uncond + cfg_scale * (eps_cond - eps_uncond)      (eps_cond alone when cond_row_offset == 0)
+ *     x0    = (x_pred - sigma * eps) * inv_alpha                    (data prediction at t_i, x_pred = the denoiser input)
+ *     x_c   = has_corr ? cA * x + (c0 * x0 + c1 * x0_prev) + cN * noise : x_pred        (corrector of step i)
+ *     x_pred <- pA * x_c + (p0 * x0 + p1 * x0_prev) + pN * noise_next                   (predictor of step i + 1)
+ *     x <- x_c,  x0_prev <- x0
+ * with host-computed scalars (pixart_sigma_b200/sampler.py, SASolverSampler.plan); p1 = 0 for a first-order predictor.
+ * After the last evaluation x_pred holds the sample.  Every product and sum is rounded separately, in the order above
+ * (the reference's float32 tensor ops), so only the reciprocal inv_alpha differs from it.
+ * `model_out`: the unconditional output of image j at row j, the conditional one at row j + cond_row_offset (n for the
+ * CFG batch [uncond (n) ; cond (n)], 0 for a single conditional evaluation); element (row, ch, p) at
+ * model_out[row * out_batch_stride + ch * hw + p], ch < 4 (the 8-channel learn-sigma output can be passed as is).
+ * fp32 arithmetic; x, x_pred, x0_prev, noise, noise_next: fp32 [n, 4, hw] contiguous; x, x_pred, x0_prev updated in place.
+ * x and noise are not read when has_corr == 0, x0_prev not read when has_corr == 0 and p1 == 0.
+ * HBM-bound: 40 (fp32 CFG output) / 36 (bf16) algorithmic bytes per latent element.
+ */
+typedef struct PxaSaStepArgs {
+  const void* model_out;    /* [cond_row_offset + n, >=4, hw], dtype out_dtype        */
+  float* x;                 /* fp32 [n, 4, hw] in/out: corrected state                */
+  float* x_pred;            /* fp32 [n, 4, hw] in/out: predicted state                */
+  float* x0_prev;           /* fp32 [n, 4, hw] in/out: previous data prediction       */
+  const float* noise;       /* fp32 [n, 4, hw]: noise of step i (corrector)           */
+  const float* noise_next;  /* fp32 [n, 4, hw]: noise of step i + 1 (predictor)       */
+  int64_t out_batch_stride; /* elements                                               */
+  int32_t n, hw;
+  int32_t cond_row_offset;  /* 0 or n                                                 */
+  int32_t out_dtype;        /* PXA_DTYPE_*                                            */
+  int32_t has_corr;         /* 0 at the first evaluation                              */
+  float cfg_scale, sigma, inv_alpha;
+  float cA, c0, c1, cN;     /* corrector of step i                                    */
+  float pA, p0, p1, pN;     /* predictor of step i + 1                                */
+} PxaSaStepArgs;
+int pxa_sa_solver_step(const PxaSaStepArgs* args, void* stream);
+
 /* =============================================================================================== training backward
  * The reference trains through torch autograd (train_scripts/train.py:197 `accelerator.backward(loss)`, per-block
  * activation checkpointing diffusion/model/utils.py:28-45).  The entry points below are the backward twins of the forward

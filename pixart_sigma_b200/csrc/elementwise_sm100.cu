@@ -295,6 +295,111 @@ extern "C" int pxa_dpm_solver_pp_step(const PxaDpmStepArgs* args, void* stream) 
 
 namespace pxa {
 
+// ------------------------------------------------------------------------------------------------- SA-Solver step
+// One thread per 4 consecutive latent elements (hw % 4 == 0): CFG combine + data prediction + corrector + next predictor.
+// Explicitly rounded operations (no FMA contraction) so the pass reproduces the reference's sequence of float32 tensor ops.
+struct SaStepScalars {
+  float cfg, sigma, inv_alpha, cA, c0, c1, cN, pA, p0, p1, pN;
+};
+
+PXA_DEVICE float4 ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
+
+template <typename OT>
+PXA_DEVICE void ld_out4(const OT* p, float (&v)[4]) {
+  if constexpr (sizeof(OT) == 4) {
+    const float4 u = *reinterpret_cast<const float4*>(p);
+    v[0] = u.x; v[1] = u.y; v[2] = u.z; v[3] = u.w;
+  } else {
+    const uint2 u = *reinterpret_cast<const uint2*>(p);
+    v[0] = bf16_lo(u.x); v[1] = bf16_hi(u.x); v[2] = bf16_lo(u.y); v[3] = bf16_hi(u.y);
+  }
+}
+
+// a * x + (b * y + c * z) + d * w, each product and sum rounded
+PXA_DEVICE float pc_update(float a, float x, float b, float y, float c, float z, float d, float w) {
+  return __fadd_rn(__fadd_rn(__fmul_rn(a, x), __fadd_rn(__fmul_rn(b, y), __fmul_rn(c, z))), __fmul_rn(d, w));
+}
+
+template <typename OT>
+__global__ void __launch_bounds__(256) sa_step_kernel(const OT* __restrict__ mo, float* __restrict__ x,
+                                                      float* __restrict__ xp, float* __restrict__ x0_prev,
+                                                      const float* __restrict__ noise, const float* __restrict__ noise_next,
+                                                      long long obs, int n, int hw, int cond_off, int has_corr,
+                                                      SaStepScalars s) {
+  const long long total = (long long)n * hw;                // 4 channels * hw elements / 4 per thread, per image
+  const bool read_prev = has_corr || s.p1 != 0.f;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int img = (int)(i / hw);
+    const int e = (int)(i - (long long)img * hw) * 4;        // element offset inside the image's [4, hw] block
+    float ec[4], eps[4];
+    ld_out4(mo + (size_t)(img + cond_off) * obs + e, ec);
+    if (cond_off) {
+      float eu[4];
+      ld_out4(mo + (size_t)img * obs + e, eu);
+#pragma unroll
+      for (int k = 0; k < 4; ++k) eps[k] = __fadd_rn(eu[k], __fmul_rn(s.cfg, __fsub_rn(ec[k], eu[k])));
+    } else {
+#pragma unroll
+      for (int k = 0; k < 4; ++k) eps[k] = ec[k];
+    }
+    const size_t off = (size_t)img * 4 * hw + e;
+    const float4 pv4 = ld4(xp + off), nn4 = ld4(noise_next + off);
+    float4 xv4 = pv4, nv4 = make_float4(0.f, 0.f, 0.f, 0.f), qv4 = nv4;
+    if (has_corr) { xv4 = ld4(x + off); nv4 = ld4(noise + off); }
+    if (read_prev) qv4 = ld4(x0_prev + off);
+    const float p[4] = {pv4.x, pv4.y, pv4.z, pv4.w}, nn[4] = {nn4.x, nn4.y, nn4.z, nn4.w};
+    const float xs[4] = {xv4.x, xv4.y, xv4.z, xv4.w}, nz[4] = {nv4.x, nv4.y, nv4.z, nv4.w};
+    const float q[4] = {qv4.x, qv4.y, qv4.z, qv4.w};
+    float x0[4], xc[4], xn[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      x0[k] = __fmul_rn(__fsub_rn(p[k], __fmul_rn(s.sigma, eps[k])), s.inv_alpha);
+      xc[k] = has_corr ? pc_update(s.cA, xs[k], s.c0, x0[k], s.c1, q[k], s.cN, nz[k]) : p[k];
+      xn[k] = pc_update(s.pA, xc[k], s.p0, x0[k], s.p1, q[k], s.pN, nn[k]);
+    }
+    *reinterpret_cast<float4*>(x + off) = make_float4(xc[0], xc[1], xc[2], xc[3]);
+    *reinterpret_cast<float4*>(xp + off) = make_float4(xn[0], xn[1], xn[2], xn[3]);
+    *reinterpret_cast<float4*>(x0_prev + off) = make_float4(x0[0], x0[1], x0[2], x0[3]);
+  }
+}
+
+}  // namespace pxa
+
+extern "C" int pxa_sa_solver_step(const PxaSaStepArgs* args, void* stream) {
+  using namespace pxa;
+  if (!args) return fail(PXA_ERR_ARG, "null args");
+  const PxaSaStepArgs& a = *args;
+  if (!a.model_out || !a.x || !a.x_pred || !a.x0_prev || !a.noise || !a.noise_next) return fail(PXA_ERR_ARG, "null pointer");
+  if (a.n <= 0 || a.hw <= 0 || (a.hw & 3)) return fail(PXA_ERR_ARG, "n > 0 and hw a positive multiple of 4 required (n=%d hw=%d)", a.n, a.hw);
+  if (a.cond_row_offset != 0 && a.cond_row_offset != a.n) return fail(PXA_ERR_ARG, "cond_row_offset must be 0 or n");
+  if (a.out_batch_stride < 4LL * a.hw) return fail(PXA_ERR_ARG, "out_batch_stride smaller than 4*hw");
+  if (a.out_dtype != PXA_DTYPE_F32 && a.out_dtype != PXA_DTYPE_BF16) return fail(PXA_ERR_ARG, "out_dtype must be PXA_DTYPE_F32 or PXA_DTYPE_BF16");
+  const int esz = a.out_dtype == PXA_DTYPE_F32 ? 4 : 2;
+  if ((reinterpret_cast<uintptr_t>(a.model_out) & (4 * esz - 1)) || ((a.out_batch_stride * esz) & (4 * esz - 1)) ||
+      ((reinterpret_cast<uintptr_t>(a.x) | reinterpret_cast<uintptr_t>(a.x_pred) | reinterpret_cast<uintptr_t>(a.x0_prev) |
+        reinterpret_cast<uintptr_t>(a.noise) | reinterpret_cast<uintptr_t>(a.noise_next)) & 15))
+    return fail(PXA_ERR_ALIGN, "model_out / x / x_pred / x0_prev / noise / noise_next must be aligned to 4 elements");
+  PXA_REQUIRE_SM100();
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  const long long total = (long long)a.n * a.hw;
+  int grid = (int)((total + 255) / 256);
+  const int cap = device_info().sms * 8;
+  if (grid > cap) grid = cap;
+  const SaStepScalars sc{a.cfg_scale, a.sigma, a.inv_alpha, a.cA, a.c0, a.c1, a.cN, a.pA, a.p0, a.p1, a.pN};
+  if (a.out_dtype == PXA_DTYPE_F32)
+    sa_step_kernel<float><<<grid, 256, 0, s>>>(reinterpret_cast<const float*>(a.model_out), a.x, a.x_pred, a.x0_prev, a.noise,
+                                               a.noise_next, a.out_batch_stride, a.n, a.hw, a.cond_row_offset, a.has_corr, sc);
+  else
+    sa_step_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16*>(a.model_out), a.x, a.x_pred,
+                                                       a.x0_prev, a.noise, a.noise_next, a.out_batch_stride, a.n, a.hw,
+                                                       a.cond_row_offset, a.has_corr, sc);
+  launch_counter()++;
+  PXA_CHECK_CUDA(cudaGetLastError());
+  return PXA_OK;
+}
+
+namespace pxa {
+
 // ------------------------------------------------------------------------------------------------- fused-LN chain: first link
 // a = bf16(x * mult[b]) with mult = 1 + scale, stats[row][0] = (sum x, sum x^2), stats[row][1..] = 0 (see PXA_EPI_LN_BIAS).
 // One warp per row like ln_modulate: reads x once (fp32), writes a once (bf16): (4 + 2) * C bytes per row.

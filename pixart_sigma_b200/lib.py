@@ -104,6 +104,15 @@ class DpmStepArgs(C.Structure):
                 ("a", C.c_float), ("b", C.c_float), ("c", C.c_float)]
 
 
+class SaStepArgs(C.Structure):
+    _fields_ = [("model_out", C.c_void_p), ("x", C.c_void_p), ("x_pred", C.c_void_p), ("x0_prev", C.c_void_p),
+                ("noise", C.c_void_p), ("noise_next", C.c_void_p), ("out_batch_stride", C.c_int64),
+                ("n", C.c_int32), ("hw", C.c_int32), ("cond_row_offset", C.c_int32), ("out_dtype", C.c_int32),
+                ("has_corr", C.c_int32), ("cfg_scale", C.c_float), ("sigma", C.c_float), ("inv_alpha", C.c_float),
+                ("cA", C.c_float), ("c0", C.c_float), ("c1", C.c_float), ("cN", C.c_float),
+                ("pA", C.c_float), ("p0", C.c_float), ("p1", C.c_float), ("pN", C.c_float)]
+
+
 class GateResidualArgs(C.Structure):
     _fields_ = [("x", C.c_void_p), ("y", C.c_void_p), ("gate", C.c_void_p), ("out", C.c_void_p), ("dgate", C.c_void_p),
                 ("gate_batch_stride", C.c_int64), ("rows_per_batch", C.c_int32), ("M", C.c_int32), ("C", C.c_int32)]
@@ -140,7 +149,7 @@ EXPORTS = ("pxa_transpose_bf16", "pxa_gelu_tanh_bf16", "pxa_gate_residual_fwd", 
            "pxa_version", "pxa_last_error", "pxa_launch_count", "pxa_gemm_bf16", "pxa_ln_modulate",
            "pxa_flash_attn_d72_bf16", "pxa_kv_compress_conv2_ln", "pxa_conv3x3_nhwc_bf16", "pxa_dpm_solver_pp_step",
            "pxa_ln_prepare", "pxa_layernorm_affine_bf16", "pxa_groupnorm_silu_nhwc_bf16", "pxa_adamw_flat", "pxa_mlp_fused_bf16",
-           "pxa_rmsnorm_bf16", "pxa_t5_attn_d64_bf16")
+           "pxa_rmsnorm_bf16", "pxa_t5_attn_d64_bf16", "pxa_sa_solver_step")
 
 _lib = None
 
@@ -158,7 +167,7 @@ def load() -> C.CDLL:
         for name, struct in (("pxa_gemm_bf16", GemmArgs), ("pxa_ln_modulate", LnModArgs),
                              ("pxa_flash_attn_d72_bf16", AttnArgs), ("pxa_kv_compress_conv2_ln", KvCompressArgs),
                              ("pxa_conv3x3_nhwc_bf16", Conv3x3Args), ("pxa_dpm_solver_pp_step", DpmStepArgs),
-                             ("pxa_ln_prepare", LnPrepareArgs), ("pxa_adamw_flat", AdamWArgs),
+                             ("pxa_sa_solver_step", SaStepArgs), ("pxa_ln_prepare", LnPrepareArgs), ("pxa_adamw_flat", AdamWArgs),
                              ("pxa_mlp_fused_bf16", MlpArgs), ("pxa_t5_attn_d64_bf16", T5AttnArgs)):
             fn = getattr(lib, name)
             fn.restype = C.c_int
@@ -458,6 +467,28 @@ def dpm_solver_pp_step(model_out: torch.Tensor, x: torch.Tensor, x0_prev: torch.
                        inv_alpha_s=1.0 / alpha_s, a=a, b=b, c=c)
     _check(load().pxa_dpm_solver_pp_step(C.byref(args), _stream()), "pxa_dpm_solver_pp_step")
     return x
+
+
+def sa_solver_step(model_out: torch.Tensor, x: torch.Tensor, x_pred: torch.Tensor, x0_prev: torch.Tensor, noise: torch.Tensor,
+                   noise_next: torch.Tensor, *, guided: bool, cfg_scale: float, sigma: float, inv_alpha: float, has_corr: bool,
+                   cA: float, c0: float, c1: float, cN: float, pA: float, p0: float, p1: float, pN: float) -> torch.Tensor:
+    """One SA-Solver evaluation step (corrector of step i, predictor of step i + 1), in place on x, x_pred and x0_prev
+    (include/pixart_sm100.h: pxa_sa_solver_step).  model_out: denoiser output, (2n, C>=4, h, w) [uncond; cond] when guided,
+    else (n, C>=4, h, w), fp32 or bf16 -- a channel-sliced view of the 8-channel learn-sigma output is fine; the state and
+    noise tensors: fp32 (n, 4, h, w) contiguous."""
+    for t in (x, x_pred, x0_prev, noise, noise_next):
+        assert t.is_cuda and t.dtype == torch.float32 and t.is_contiguous() and t.shape == x.shape
+    assert model_out.is_cuda and x.dim() == 4 and x.shape[1] == 4
+    n, _, h, w = x.shape
+    assert model_out.shape[0] == (2 * n if guided else n) and model_out.shape[1] >= 4 and model_out.shape[2:] == (h, w)
+    assert model_out.stride(3) == 1 and model_out.stride(2) == w and model_out.stride(1) == h * w, "model_out: (.., h, w) planes must be dense"
+    args = SaStepArgs(model_out=_ptr(model_out), x=_ptr(x), x_pred=_ptr(x_pred), x0_prev=_ptr(x0_prev), noise=_ptr(noise),
+                      noise_next=_ptr(noise_next), out_batch_stride=model_out.stride(0), n=n, hw=h * w,
+                      cond_row_offset=n if guided else 0, out_dtype=_dt(model_out.dtype), has_corr=int(bool(has_corr)),
+                      cfg_scale=cfg_scale, sigma=sigma, inv_alpha=inv_alpha, cA=cA, c0=c0, c1=c1, cN=cN, pA=pA, p0=p0,
+                      p1=p1, pN=pN)
+    _check(load().pxa_sa_solver_step(C.byref(args), _stream()), "pxa_sa_solver_step")
+    return x_pred
 
 
 # ------------------------------------------------------------------------------------------------- training backward

@@ -892,10 +892,11 @@ def install_into_reference() -> bool:
         setattr(nets, name, obj)
     nets.PixArtMSBlock = PixArtMSBlock
     nets.PixArtBlock = PixArtBlock
-    try:                                                   # the sampler the inference script imports from `diffusion`
+    try:                                                   # the samplers the inference script imports from `diffusion`
         import diffusion
-        from .sampler import DPMS
+        from .sampler import DPMS, SASolverSampler
         diffusion.DPMS = DPMS
+        diffusion.SASolverSampler = SASolverSampler
     except Exception:
         pass
     return True

@@ -1,4 +1,4 @@
-"""B200-native driver of the DPM-Solver++ sampling loop around the denoiser hot path (SURVEY.md §8f.1).
+"""B200-native drivers of the DPM-Solver++ and SA-Solver sampling loops around the denoiser hot path (SURVEY.md §8f.1).
 
 Mirrors the reference's `diffusion.DPMS(...)` factory and `DPM_Solver.sample(...)` as `scripts/inference.py:102-118` uses
 them (`diffusion/dpm_solver.py:6-35`, `diffusion/model/dpm_solver.py:1069-1241`): same call signature, same result, for
@@ -13,6 +13,9 @@ What is different from the reference loop:
     step (`pxa_dpm_solver_pp_step`, include/pixart_sm100.h) instead of ~25 PyTorch elementwise launches;
   * `cuda_graph=True` captures the whole `steps`-step loop (denoiser launches included) into one CUDA graph.
 There is no CPU path: inputs must live on an sm_100 device.
+
+`SASolverSampler` does the same for the reference's `diffusion.SASolverSampler` (`--sampling_algo sa-solver`,
+scripts/inference.py:119-133) with one fused predictor-corrector kernel per denoiser evaluation (`pxa_sa_solver_step`).
 """
 from __future__ import annotations
 
@@ -23,7 +26,7 @@ import torch
 
 from . import lib
 
-__all__ = ["DPMS", "DPMSolverPP"]
+__all__ = ["DPMS", "DPMSolverPP", "SASolverSampler"]
 
 
 class _DiscreteVPSchedule:
@@ -59,6 +62,33 @@ class _DiscreteVPSchedule:
     def lam(self, t):
         la = self.log_alpha_at(t)
         return la - 0.5 * torch.log(1. - torch.exp(2. * la))
+
+
+class _AlphasCumprodSchedule(_DiscreteVPSchedule):
+    """The same look-ups over the table `NoiseScheduleVP('discrete', alphas_cumprod=...)` builds for the SA-Solver wrapper:
+    log(alpha) = 0.5 log(alphas_cumprod) with alphas_cumprod = float32(cumprod(1 - linear betas)), the logarithm taken in
+    float32, no log-SNR clipping (diffusion/sa_sampler.py:19-22, diffusion/model/sa_solver.py:81-90)."""
+
+    def __init__(self, diffusion_steps: int = 1000):
+        scale = 1000 / diffusion_steps
+        betas = np.linspace(scale * 0.0001, scale * 0.02, diffusion_steps, dtype=np.float64)
+        alphas_cumprod = torch.cumprod(1.0 - torch.from_numpy(betas), dim=0).to(torch.float32)
+        self.log_alpha = 0.5 * torch.log(alphas_cumprod)
+        self.total_N = self.log_alpha.numel()
+        self.t = torch.linspace(0., 1., self.total_N + 1)[1:].to(torch.float32)
+        self.T = 1.0
+
+
+def _captured_model_key(model: Callable, params: List[torch.Tensor], model_kwargs: dict) -> tuple:
+    """What a captured denoiser call depends on beyond its inputs: the model_kwargs tensors (captured by address) and, when the
+    forward keeps derived copies of its weights (stacked kv_linear weights, fused-LN tables) that a replay cannot refresh, the
+    parameters' versions."""
+    kw_id = tuple(sorted((k, (v.data_ptr(), tuple(v.shape)) if isinstance(v, torch.Tensor) else repr(v))
+                         for k, v in (model_kwargs or {}).items()))
+    owner = getattr(model, "__self__", model)
+    derived = getattr(owner, "_kv_batch", None) is not None or getattr(owner, "_ln_fusion", None) is not None
+    wkey = (sum(p._version for p in params), params[0].data_ptr()) if (params and derived) else None
+    return kw_id, wkey
 
 
 class DPMSolverPP:
@@ -155,13 +185,8 @@ class DPMSolverPP:
     def _sample_graphed(self, x, plan, t_dev, cond):
         # every per-step scalar (sigma_s, alpha_s, a, b, c), the step orders and t_input are baked into the captured kernel
         # arguments, and `cond` / model_kwargs tensors into the captured forward: all of them are part of the key
-        kw_id = tuple(sorted((k, (v.data_ptr(), tuple(v.shape)) if isinstance(v, torch.Tensor) else repr(v))
-                             for k, v in (self.model_kwargs or {}).items()))
-        # ... and so are the denoiser's parameters: the forward keeps derived copies (stacked kv_linear weights) a replay cannot refresh
-        owner = getattr(self.model, "__self__", self.model)
-        derived = getattr(owner, "_kv_batch", None) is not None or getattr(owner, "_ln_fusion", None) is not None
-        wkey = (sum(p._version for p in self._params), self._params[0].data_ptr()) if (self._params and derived) else None
-        key = (tuple(x.shape), x.device.index, float(self.cfg_scale), cond.data_ptr(), tuple(cond.shape), kw_id, wkey,
+        key = (tuple(x.shape), x.device.index, float(self.cfg_scale), cond.data_ptr(), tuple(cond.shape),
+               _captured_model_key(self.model, self._params, self.model_kwargs),
                tuple((st["t_input"], st["sigma_s"], st["alpha_s"], st["a"], st["b"], st["c"], st.get("order")) for st in plan))
         if key not in self._graphs:
             x_static = x.to(torch.float32).contiguous().clone()
@@ -191,3 +216,180 @@ def DPMS(model: Callable, condition: torch.Tensor, uncondition: Optional[torch.T
         raise NotImplementedError("only model_type='noise', noise_schedule='linear', guidance_type='classifier-free' "
                                   "(what scripts/inference.py uses)")
     return DPMSolverPP(model, condition, uncondition, cfg_scale, model_kwargs, diffusion_steps)
+
+
+# ------------------------------------------------------------------------------------------------- SA-Solver
+def _exp_integral(order: int, start, end, tau):
+    """int_start^end exp(x (1 + tau^2)) x^order dx for order 0 / 1 (diffusion/model/sa_solver.py:449-471)."""
+    k = 1 + tau ** 2
+    end_c, start_c = k * end, k * start
+    if order == 0:
+        return torch.exp(end_c) * (1 - torch.exp(-(end_c - start_c))) / k
+    return torch.exp(end_c) * ((end_c - 1) - (start_c - 1) * torch.exp(-(end_c - start_c))) / (k ** 2)
+
+
+def _sa_update(sch: _DiscreteVPSchedule, order: int, tau, t_prev: List[torch.Tensor], t: torch.Tensor, corrector: bool):
+    """(A, [g0, g1], N) of x_new = A x + g0 m[-1] + g1 m[-2] + N noise for the data-prediction SA predictor (corrector=False)
+    or corrector of `order` 1 / 2 with the "few steps" term (diffusion/model/sa_solver.py:478-560,644-753), as float32 (1,)
+    tensors computed by the reference's operations in the reference's order."""
+    sigma_t, lam_t = sch.sigma(t), sch.lam(t)
+    lam_prev = sch.lam(t_prev[-1])
+    h = lam_t - lam_prev
+    nodes = (t_prev + [t]) if corrector else t_prev
+    if order == 1:
+        lagrange = [[1]]
+    else:
+        l0, l1 = sch.lam(nodes[-1]), sch.lam(nodes[-2])
+        lagrange = [[1 / (l0 - l1), -l1 / (l0 - l1)], [1 / (l1 - l0), -l0 / (l1 - l0)]]
+    g = []
+    for i in range(order):
+        c = 0
+        for j in range(order):
+            c += lagrange[i][j] * _exp_integral(order - 1 - j, lam_prev, lam_t, tau)
+        g.append(c)
+    if order == 2:
+        k = 1 + tau ** 2
+        if corrector:
+            extra = 1.0 * torch.exp(k * lam_t) * (h / 2 - (h * k - 1 + torch.exp(k * (-h))) / (k ** 2 * h))
+        else:
+            extra = 1.0 * torch.exp(k * lam_t) * (h ** 2 / 2 - (h * k - 1 + torch.exp(k * (-h))) / (k ** 2)) / (
+                lam_prev - sch.lam(t_prev[-2]))
+        g = [g[0] + extra, g[1] - extra]
+    g = [(1 + tau ** 2) * sigma_t * torch.exp(- tau ** 2 * lam_t) * gi for gi in g]
+    A = torch.exp(-tau ** 2 * h) * (sigma_t / sch.sigma(t_prev[-1]))
+    N = sigma_t * torch.sqrt(1 - torch.exp(-2 * tau ** 2 * h))
+    return A, g, N
+
+
+class SASolverSampler:
+    """The SA-Solver sampler of `diffusion.SASolverSampler` (diffusion/sa_sampler.py) on the sm_100a step kernel.
+
+    Same constructor and `.sample(...)` signature and the same result as the reference wrapper, which always runs
+    `SASolver(algorithm_type="data_prediction").sample(mode='few_steps', skip_type='time', skip_order=1, predictor_order=2,
+    corrector_order=2, pc_mode='PEC', tau=lambda t: eta if 0.2 <= t <= 0.8 else 0)` around the noise-prediction model with
+    classifier-free guidance.  The loop makes S denoiser evaluations and S + 1 standard-normal draws (the first one unused,
+    the last one scaled by tau = 0), in the reference's order from the default CUDA generator, so a seeded run consumes the
+    generator as the reference would.
+
+    What is different from the reference loop: every schedule look-up and coefficient (each an `interpolate_fn` that sorts a
+    1001-element array on the GPU in the reference, ~25-30 per step, plus a host sync for tau(t)) is computed once on the
+    host by `plan`; the CFG combine, data prediction, corrector and next predictor are ONE elementwise kernel per evaluation
+    (`pxa_sa_solver_step`, include/pixart_sm100.h); `cuda_graph=True` captures the noise draws and every denoiser and step
+    launch of the loop into one CUDA graph.  There is no CPU path."""
+
+    def __init__(self, model: Callable, noise_schedule="linear", diffusion_steps=1000, device='cpu'):
+        if noise_schedule != "linear":
+            raise NotImplementedError("only noise_schedule='linear' (what scripts/inference.py uses)")
+        self.model = model
+        self.device = device
+        self.schedule = _AlphasCumprodSchedule(diffusion_steps)
+        self._graphs: Dict[tuple, tuple] = {}
+        owner = getattr(model, "__self__", model)              # the nn.Module behind a bound forward_with_dpmsolver
+        self._params = list(owner.parameters()) if isinstance(owner, torch.nn.Module) else []
+
+    # ---- host side: everything that does not depend on the latents
+    def plan(self, S: int, eta) -> List[dict]:
+        """Per denoiser evaluation i at time ts[i], ts = linspace(1, 1/N, S + 1): the model-input time and the scalars of
+        pxa_sa_solver_step -- sigma, 1/alpha at ts[i]; the corrector of step i (has_corr, cA, c0, c1, cN; tau_c) and the
+        predictor of step i + 1 (pA, p0, p1, pN; tau_p; order 1 at the first and last step, else 2; tau = 0 at the last)."""
+        if S < 2:
+            raise ValueError(f"S must be >= 2 (the predictor / corrector orders are 2), got {S}")
+        sch = self.schedule
+        ts = torch.linspace(sch.T, 1. / sch.total_N, S + 1)               # skip_type='time', skip_order=1
+        tau = lambda t: eta if 0.2 <= t <= 0.8 else 0                     # float32 t against 0.2 / 0.8, as the reference
+        plan = []
+        for i in range(S):
+            t = ts[i]
+            st = dict(t_input=float((t - 1. / sch.total_N) * 1000.), sigma=float(sch.sigma(t)), inv_alpha=float(1. / sch.alpha(t)),
+                      has_corr=i >= 1, tau_c=0, cA=0., c0=0., c1=0., cN=0.)
+            if i >= 1:
+                st["tau_c"] = tau(t)
+                A, (c0, c1), N = _sa_update(sch, 2, st["tau_c"], [ts[j] for j in range(max(0, i - 2), i)], t, True)
+                st.update(cA=float(A), c0=float(c0), c1=float(c1), cN=float(N))
+            step = i + 1
+            order = 1 if step in (1, S) else 2
+            st["tau_p"] = 0 if step == S else tau(ts[step])
+            A, g, N = _sa_update(sch, order, st["tau_p"], [ts[j] for j in range(max(0, i - 1), i + 1)], ts[step], False)
+            st.update(pA=float(A), p0=float(g[0]), p1=float(g[1]) if order == 2 else 0., pN=float(N), order=order)
+            plan.append(st)
+        return plan
+
+    # ---- device side
+    def _draw(self, buf: torch.Tensor) -> None:
+        """One of the loop's standard-normal draws (the reference's `torch.randn_like(x)`), into `buf`."""
+        buf.normal_()
+
+    def _run(self, x, x_pred, x0_prev, noise, plan, t_dev, cond, guided, cfg, model_kwargs, draw) -> torch.Tensor:
+        draw(noise[0])                                   # the reference draws once before the first evaluation, unused
+        for i, (st, t_in) in enumerate(zip(plan, t_dev)):
+            out = self.model(torch.cat([x_pred, x_pred]) if guided else x_pred, t_in, cond, **model_kwargs)
+            if out.dtype not in (torch.float32, torch.bfloat16):
+                out = out.float()
+            if not (out.stride(3) == 1 and out.stride(2) == out.shape[3] and out.stride(1) == out.shape[2] * out.shape[3]):
+                out = out.contiguous()
+            draw(noise[(i + 1) % 2])                     # the noise of step i + 1, drawn after evaluation i as in the reference
+            lib.sa_solver_step(out, x, x_pred, x0_prev, noise[i % 2], noise[(i + 1) % 2], guided=guided, cfg_scale=cfg,
+                               sigma=st["sigma"], inv_alpha=st["inv_alpha"], has_corr=st["has_corr"], cA=st["cA"],
+                               c0=st["c0"], c1=st["c1"], cN=st["cN"], pA=st["pA"], p0=st["p0"], p1=st["p1"], pN=st["pN"])
+        return x_pred
+
+    @torch.no_grad()
+    def sample(self, S, batch_size, shape, conditioning=None, callback=None, normals_sequence=None, img_callback=None,
+               quantize_x0=False, eta=0., mask=None, x0=None, temperature=1., noise_dropout=0., score_corrector=None,
+               corrector_kwargs=None, verbose=True, x_T=None, log_every_t=100, unconditional_guidance_scale=1.,
+               unconditional_conditioning=None, model_kwargs={}, *, cuda_graph=False, **kwargs):
+        """Returns (x, None), x the fp32 sample of shape x_T.shape.  Like the reference, the arguments between `callback`
+        and `log_every_t` other than `eta`, `x_T` are accepted and ignored.  x_T None: drawn with
+        `torch.randn((batch_size,) + shape, device=device)` first.  cuda_graph=True: capture the loop once per configuration
+        and replay it (x_T is drawn outside the graph; each replay draws fresh noise from the generator)."""
+        plan = self.plan(S, eta)
+        C, H, W = shape
+        if x_T is None:
+            if torch.device(self.device).type != "cuda":
+                raise RuntimeError("pixart_sigma_b200.sampler has no CPU path: construct SASolverSampler with a CUDA device")
+            x_T = torch.randn((batch_size, C, H, W), device=self.device)
+        if not x_T.is_cuda:
+            raise RuntimeError("pixart_sigma_b200.sampler has no CPU path: x_T must be a CUDA tensor")
+        if x_T.dim() != 4 or x_T.shape[1] != 4 or (x_T.shape[2] * x_T.shape[3]) % 4:
+            raise ValueError("latents must be (n, 4, h, w) with h*w a multiple of 4")
+        if x_T.dtype != torch.float32:
+            raise ValueError("x_T must be float32 (the loop's noise draws take its dtype)")
+        guided = not (unconditional_guidance_scale == 1. or unconditional_conditioning is None)
+        cond = torch.cat([unconditional_conditioning, conditioning]) if guided else conditioning    # [uncond ; cond]
+        rows = 2 * x_T.shape[0] if guided else x_T.shape[0]
+        t_dev = [torch.full((rows,), st["t_input"], dtype=torch.float32, device=x_T.device) for st in plan]
+        cfg = float(unconditional_guidance_scale) if guided else 1.0
+        if cuda_graph:
+            return self._sample_graphed(x_T, plan, t_dev, cond, guided, cfg, model_kwargs, S, eta), None
+        x_pred = x_T.contiguous().clone()
+        x, x0_prev = torch.empty_like(x_pred), torch.empty_like(x_pred)
+        noise = [torch.empty_like(x_pred), torch.empty_like(x_pred)]
+        return self._run(x, x_pred, x0_prev, noise, plan, t_dev, cond, guided, cfg, model_kwargs, self._draw), None
+
+    def _sample_graphed(self, x_T, plan, t_dev, cond, guided, cfg, model_kwargs, S, eta):
+        # the plan's scalars and t_input are baked into the captured kernel arguments and the model_kwargs tensors into the
+        # captured forward (by address): all of them are part of the key.  x_T and the conditioning (a new tensor per call)
+        # are copied into the graph's own input buffers.
+        key = (tuple(x_T.shape), x_T.device.index, guided, cfg, tuple(cond.shape), cond.dtype,
+               _captured_model_key(self.model, self._params, model_kwargs), S, eta,
+               tuple(tuple(v for k, v in sorted(st.items())) for st in plan))
+        if key not in self._graphs:
+            bufs = [torch.empty_like(x_T) for _ in range(6)]               # z_in, x, x_pred, x0_prev, 2 x noise
+            z_in, x, x_pred, x0_prev = bufs[:4]
+            cond_in = cond.clone()
+            side = torch.cuda.Stream()
+            side.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(side):        # warm-up outside capture (lazy inits), zero noise: the generator is untouched
+                x_pred.copy_(x_T)
+                self._run(x, x_pred, x0_prev, bufs[4:], plan[:2], t_dev[:2], cond_in, guided, cfg, model_kwargs, torch.Tensor.zero_)
+            torch.cuda.current_stream().wait_stream(side)
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):
+                x_pred.copy_(z_in)
+                self._run(x, x_pred, x0_prev, bufs[4:], plan, t_dev, cond_in, guided, cfg, model_kwargs, self._draw)
+            self._graphs[key] = (graph, z_in, cond_in, x_pred, bufs, t_dev)
+        graph, z_in, cond_in, x_pred = self._graphs[key][:4]
+        z_in.copy_(x_T)
+        cond_in.copy_(cond)
+        graph.replay()
+        return x_pred.clone()
